@@ -107,16 +107,15 @@ def _ref_arm():
 
 def run_reference(args, rank):
     """`--impl reference`: the reference's own training iteration on the host cores (unmodified modules from
-    baseline/_ref/reference when present, else the oracle port), bounded sample."""
+    oracle/_ref when present, else the oracle port), `--steps` timed iterations after `--warmup` untimed ones."""
     if rank != 0:
         return
-    steps, warmup = max(1, min(args.steps, 5)), max(1, min(args.warmup, 2))
-    r = _ref_arm().cpu_train_baseline(steps, warmup, PER_GPU_BATCH)
+    r = _ref_arm().cpu_train_baseline(args.steps, args.warmup, PER_GPU_BATCH)
     out = {'metric': METRIC, 'value': r['value'], 'unit': 'samples/s', 'n_gpus': args.gpus, 'steps': r['steps'],
-           'warmup': warmup, 'ms_per_step': r['ms_per_step'], 'higher_is_better': True, 'scaling': 'weak',
+           'warmup': args.warmup, 'ms_per_step': r['ms_per_step'], 'higher_is_better': True, 'scaling': 'weak',
            'vs_baseline': None, 'dtype': 'f32', 'data': 'synthetic', 'impl': 'reference',
            'config': {'workload': 'Darcy 64x64 PIDM train step (mean-mode x0), Unet3D dim=32, batch 32, host CPU',
-                      'global_batch': PER_GPU_BATCH, 'note': 'bounded sample: steps/warmup clamped to <=5/<=2'},
+                      'global_batch': PER_GPU_BATCH},
            'cpu_baseline': {k: r[k] for k in ('value', 'unit', 'cores', 'kind', 'sample')},
            'e2e': {'value': r['value'], 'unit': 'samples/s', 'h2d_bytes_per_step': 0, 'd2h_bytes_per_step': 0},
            'gpu_launches': 0}
@@ -425,11 +424,39 @@ def residual_kernel_sweep(pk):
                                         'ms_per_launch': res['loss']['ms'], 'algorithmic_bytes': res['loss']['bytes']}}
 
 
+DUMP_SAMPLE = 1 << 22      # sampled parameter positions: params + EMA = 2 x 16.8 MB of float32
+
+
+def dump_step_outputs(path, eng, out):
+    """`--dump-outputs DIR`: what the last timed step handed its caller, as DIR/<name>.npy in float32 -- the values
+    TrainEngine.step returns (loss, data_loss, residual_abs_mean) and the weights it left in the model (params_sample,
+    and their EMA shadow ema_sample).  The weights are the trainable parameters flattened in named_parameters() order
+    and sampled at DUMP_SAMPLE fixed positions (seeded, ascending), so that two builds can be compared position by
+    position.  The inputs are the same in every run, but weight gradients are summed with fp32 atomics and the
+    optimizer steps before the dump amplify that rounding: two runs of `--steps 20 --warmup 5` on one B200 (1000 W
+    power limit) agreed to 0.3 % in the loss and 1e-3 in the weights.  Call before any further step: the returned
+    tensors are the graph's static outputs."""
+    import numpy as np
+    named = [(n, p) for n, p in eng.model.named_parameters() if p.requires_grad]
+    ema = eng.ema_state_dict()
+    n_total = sum(p.numel() for _, p in named)
+    idx = torch.randperm(n_total, generator=torch.Generator().manual_seed(0))[:DUMP_SAMPLE].sort().values
+    idx = idx.to(out[0].device)
+    arrays = dict(zip(('loss', 'data_loss', 'residual_abs_mean'), out))
+    arrays['params_sample'] = torch.cat([p.detach().reshape(-1) for _, p in named])[idx]
+    arrays['ema_sample'] = torch.cat([ema[n].reshape(-1) for n, _ in named])[idx]
+    os.makedirs(path, exist_ok=True)
+    for name, t in arrays.items():
+        np.save(os.path.join(path, name + '.npy'), t.detach().float().cpu().numpy())
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument('--gpus', type=int, default=1)
     ap.add_argument('--steps', type=int, default=20)
     ap.add_argument('--warmup', type=int, default=5)
+    ap.add_argument('--dump-outputs', metavar='DIR', default=None,
+                    help='write what the last timed step computed to DIR/<name>.npy (b200 arm)')
     ap.add_argument('--impl', default='b200', choices=['b200', 'reference', 'cpu_extras', 'torch_cuda'])
     ap.add_argument('--no-torch-cuda-baseline', action='store_true')
     ap.add_argument('--no-graph', action='store_true')
@@ -437,6 +464,10 @@ def main():
     ap.add_argument('--no-sampling', action='store_true')
     ap.add_argument('--no-mechanics', action='store_true')
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
+    if args.dump_outputs and args.impl != 'b200':
+        ap.error('--dump-outputs applies to the b200 arm')
     rank = int(os.environ.get('RANK', '0'))
     local_rank = int(os.environ.get('LOCAL_RANK', '0'))
     world = int(os.environ.get('WORLD_SIZE', '1'))
@@ -504,6 +535,8 @@ def main():
     ms = e0.elapsed_time(e1)
     last_loss = float(out[0].item())
     log(f'device-resident: {ms / args.steps:.3f} ms/step')
+    if args.dump_outputs and rank == 0:
+        dump_step_outputs(args.dump_outputs, eng, out)
     # ---- end to end: pinned host batch -> H2D -> step -> D2H loss, every step ------------------------------------
     for _ in range(3):
         x0_dev.copy_(x0_host, non_blocking=True)

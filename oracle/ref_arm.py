@@ -7,10 +7,9 @@ oracle/ref_shims/ (SURVEY.md section 8c: einops_exts, rotary_embedding_torch, fi
 * on the B200 through stock PyTorch-CUDA (cuDNN / cuBLAS) -> the `torch_cuda_baseline` block, the comparison point
   SURVEY 2b / BASELINE.md 3.7 ask for (the reference ships no GPU kernels of its own)
 
-The reference sources are NOT part of this repository: `__graft_entry__.build()` copies /root/reference/{src,*.py,
-model.yaml} into the git-ignored baseline/_ref/reference/ when /root/reference exists (build container); the directory
-travels to the GPU box with the snapshot.  When it is absent every function here falls back to the oracle port
-(oracle/pidm_oracle.py, kind = "port") and says so.
+The reference sources are NOT part of this repository: `__graft_entry__.build()` copies them into the git-ignored
+oracle/_ref/ when the original project is at hand (oracle/fetch_reference.py).  When oracle/_ref/ is absent every
+function here falls back to the oracle port (oracle/pidm_oracle.py, kind = "port") and says so.
 
 This module must be loaded BY FILE PATH in a process whose sys.path does not contain the repo root: the repo's `src/`
 drop-in package (a regular package) would shadow the reference's `src/` (a namespace package) regardless of order.
@@ -23,7 +22,7 @@ import warnings
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(HERE)
-REF_DIR = os.path.join(ROOT, 'baseline', '_ref', 'reference')
+REF_DIR = os.path.join(HERE, '_ref')
 
 
 def reference_available():
@@ -172,9 +171,8 @@ def build_port_step(device, batch, channels_last=False):
     return step
 
 
-def time_steps(step, device, steps, warmup, budget_s=None, sync_each=True):
+def time_steps(step, device, steps, warmup, sync_each=True):
     import torch
-    t_begin = time.perf_counter()
     for _ in range(warmup):
         step()
     times = []
@@ -184,24 +182,22 @@ def time_steps(step, device, steps, warmup, budget_s=None, sync_each=True):
             if sync_each and str(device).startswith('cuda'):
                 float(out)                              # the loop reads the loss (pbar / logging)
         times.append(tm.seconds)
-        if budget_s is not None and time.perf_counter() - t_begin > budget_s:
-            break
     return times
 
 
-def cpu_train_baseline(steps, warmup, batch=32, budget_s=150.0):
+def cpu_train_baseline(steps, warmup, batch=32):
     import torch
     ncores = usable_cores()
     torch.set_num_threads(ncores)
     if reference_available():
         ref = load_reference()
         step, *_ = build_reference_step(ref, 'cpu', batch)
-        kind, what = 'reference', 'unmodified reference modules (baseline/_ref/reference/src) + import shims'
+        kind, what = 'reference', 'unmodified reference modules (oracle/_ref/src) + import shims'
     else:
         step = build_port_step('cpu', batch)
-        kind, what = 'port', 'oracle/pidm_oracle.py restatement (baseline/_ref/reference is absent on this box)'
+        kind, what = 'port', 'oracle/pidm_oracle.py restatement (oracle/_ref is absent)'
     log(f'cpu train baseline: kind={kind}, {ncores} usable cores (os.cpu_count()={os.cpu_count()}), batch {batch}')
-    times = time_steps(step, 'cpu', steps, warmup, budget_s, sync_each=False)
+    times = time_steps(step, 'cpu', steps, warmup, sync_each=False)
     sec = sum(times) / len(times)
     return dict(value=batch / sec, unit='samples/s', cores=ncores, kind=kind, ms_per_step=sec * 1e3, steps=len(times),
                 sample=f'{len(times)} training iterations (main.py:157-183 body: loss, backward, clip, Adam, EMA) at batch '
@@ -216,7 +212,7 @@ def cpu_extras(budget_s=120.0):
     torch.set_num_threads(ncores)
     out = {'cores': ncores}
     if not reference_available():
-        out['unavailable'] = 'baseline/_ref/reference is absent on this box'
+        out['unavailable'] = 'oracle/_ref is absent'
         return out
     ref = load_reference()
     _, model, diff, res = build_reference_step(ref, 'cpu', 2)
@@ -295,7 +291,7 @@ def torch_cuda_baselines(batch=32, steps=10, warmup=3):
             note='torch.autocast(bfloat16) around the whole iteration; the residual operator then also runs in bf16 for '
                  'its conv2d stencils, which the reference never does -- speed only, not a valid training setup')
     else:
-        out['reference'] = {'unavailable': 'baseline/_ref/reference is absent on this box'}
+        out['reference'] = {'unavailable': 'oracle/_ref is absent'}
     set_tf32(False)
     pstep = build_port_step(dev, batch)
     run('port_eager_fp32', pstep, kind='port')

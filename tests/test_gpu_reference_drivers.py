@@ -1,7 +1,7 @@
 """The reference's OWN driver scripts, executed against this repository's drop-in `src/` package.
 
-`baseline/_ref/reference/{main.py,main_toy.py}` are the unmodified files of the reference (fetched by
-`__graft_entry__.build()`, not part of this repository).  The scripts hard-code their run length (300,000 training
+`oracle/_ref/{main.py,main_toy.py}` are the unmodified files of the reference (copied by `__graft_entry__.build()`
+when the original project is at hand, not part of this repository; the tests skip without them).  The scripts hard-code their run length (300,000 training
 iterations, a 10^4-point data set, W&B tracking), so the test rewrites exactly those LITERALS -- listed in `EDITS` below,
 each asserted to occur -- and nothing else: imports, model construction, loss call, optimizer / clip / EMA sequence,
 sampling call, checkpoint call all execute as written by the reference's authors.  matplotlib (not installed here) is
@@ -15,7 +15,7 @@ import pytest
 
 pytestmark = pytest.mark.gpu
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF = os.path.join(ROOT, 'baseline', '_ref', 'reference')
+REF = os.path.join(ROOT, 'oracle', '_ref')
 SHIMS = os.path.join(ROOT, 'oracle', 'ref_shims')
 
 
@@ -36,7 +36,7 @@ def _edit(text, edits):
     return text
 
 
-@pytest.mark.skipif(not os.path.isfile(os.path.join(REF, 'main.py')), reason='reference scripts not fetched (baseline/_ref)')
+@pytest.mark.skipif(not os.path.isfile(os.path.join(REF, 'main.py')), reason='reference scripts not fetched (oracle/_ref)')
 def test_reference_main_py_runs_on_the_drop_in_package(tmp_path):
     """main.py (Darcy, model.yaml as shipped except diff_steps): 2 training iterations incl. validation loss, EMA,
     sampling with residual evaluation, CSV dumps and the checkpoint."""
@@ -63,7 +63,7 @@ def test_reference_main_py_runs_on_the_drop_in_package(tmp_path):
     assert 'test loss at iteration 0' in r.stdout
 
 
-@pytest.mark.skipif(not os.path.isfile(os.path.join(REF, 'main_toy.py')), reason='reference scripts not fetched (baseline/_ref)')
+@pytest.mark.skipif(not os.path.isfile(os.path.join(REF, 'main_toy.py')), reason='reference scripts not fetched (oracle/_ref)')
 def test_reference_main_toy_py_runs_on_the_drop_in_package(tmp_path):
     """main_toy.py (configs[0]): 2 epochs over a 512-point data set, sampling + CSV dump at epoch 0, checkpoint."""
     EDITS = [("'train_num_steps': 400", "'train_num_steps': 1"),
